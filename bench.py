@@ -64,7 +64,14 @@ def parse_args():
     ap.add_argument("--no-stream", action="store_true", help="N = 1: skip the streaming (configs[2]) leg")
     ap.add_argument("--stream-scans", type=int, default=40)
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="CPU baseline budget")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the cost, gradient and H of the timed evaluation as DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload in ("stream", "rgbd")):
+        ap.error("--dump-outputs applies to the registration evaluation (--impl b200, workload auto / config2 / config4)")
+    return args
 
 
 def workload_params(name, args):
@@ -667,9 +674,10 @@ class Problem:
             self.ctx.submap_free(self.id_base + sid)
 
 
-def measure(P, args, torch, dist, world, stream, want_cpu_pose_check=None):
+def measure(P, args, torch, dist, world, stream, want_cpu_pose_check=None, want_outputs=False):
     """Device-resident throughput, end-to-end call, roofline split and the pose-graph solve of one
-    resident problem.  Every rank takes part (each evaluation contains the exchange)."""
+    resident problem.  Every rank takes part (each evaluation contains the exchange).
+    want_outputs: out["outputs"] = what a caller of the timed evaluation receives (cost, gradient, H)."""
     ctx = P.ctx
 
     def barrier():
@@ -702,6 +710,11 @@ def measure(P, args, torch, dist, world, stream, want_cpu_pose_check=None):
     out["ms_per_step"] = ms_step
     out["value"] = P.r_global / (ms_step * 1e-3)
     out["gpu_launches"] = int(ctx.launch_count - launches0)
+    if want_outputs:
+        # vgx_graph_eval enqueues the evaluation each timed step enqueued, at the same poses (its sums
+        # run in a fixed order, so it repeats the last step bit for bit) and copies the result back
+        _, cost, g, H = ctx.graph_eval(P.n_nodes, want_H=True)
+        out["outputs"] = {"cost": np.array([cost]), "gradient": g, "H": H}
 
     # ---- end to end through the public call with host buffers
     e2e_steps = max(3, min(args.steps, 10))
@@ -770,6 +783,28 @@ def measure(P, args, torch, dist, world, stream, want_cpu_pose_check=None):
         ctx.graph_set_poses(P.pinit)
         out["solve"] = solve
     return out
+
+
+DUMP_LIMIT_BYTES = 60 * 10 ** 6   # array data; with the .npy headers the files stay under 64 MB
+
+
+def write_outputs(out_dir, arrays):
+    """DIR/<name>.npy (float64) per array.  A dense H too large for DUMP_LIMIT_BYTES is replaced by
+    a fixed, seeded sample of its entries: H_sample.npy (values) and H_sample_index.npy (flat
+    row-major indices, exact in float64)."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.ascontiguousarray(v, np.float64) for k, v in arrays.items()}
+    H = arrays.pop("H")
+    budget = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values())
+    if H.nbytes <= budget:
+        arrays["H"] = H
+    else:
+        n = budget // 16
+        idx = np.sort(np.random.default_rng(0).choice(H.size, n, replace=False))
+        arrays["H_sample"] = H.reshape(-1)[idx]
+        arrays["H_sample_index"] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def single_rank_parity(P, torch, dist, world, rank):
@@ -858,8 +893,10 @@ def run_b200(args):
     sampler = ClockSampler(local_rank) if rank == 0 else None
     t_load0 = time.time()
     P = Problem(ctx, api, sc)
-    M = measure(P, args, torch, dist, world, stream)
+    M = measure(P, args, torch, dist, world, stream, want_outputs=bool(args.dump_outputs))
     ms_step = M["ms_per_step"]
+    if args.dump_outputs and rank == 0:
+        write_outputs(args.dump_outputs, M.pop("outputs"))
 
     parity = None
     if world > 1:

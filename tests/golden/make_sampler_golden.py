@@ -1,8 +1,8 @@
 #!/usr/bin/env python
-"""Generates tests/golden/weighted_sampler.json from the REFERENCE's own WeightedSampler
-(oracle/_ref/libvgref_sampler.so, compiled from /root/reference/voxgraph/include/voxgraph/frontend/
-submap_collection/weighted_sampler{,_inl}.h by oracle/Makefile).  Run in the build container
-(where /root/reference exists); the fixture travels to the GPU box."""
+"""Generates tests/golden/weighted_sampler.json and tests/golden/weighted_sampler_draws.npz from the
+REFERENCE's own WeightedSampler (oracle/_ref/libvgref_sampler.so, compiled from the reference's
+include/voxgraph/frontend/submap_collection/weighted_sampler{,_inl}.h by oracle/Makefile target
+`ref`).  Needs the reference sources; the tests read only the stored fixtures."""
 import json
 import os
 import sys
@@ -32,3 +32,18 @@ json.dump({"source": "voxgraph::WeightedSampler<Item>::getRandomItem compiled fr
                      "(libstdc++ std::mt19937 + uniform_real_distribution<double>)", "cases": cases},
           open(out, "w"))
 print("wrote", out, len(cases), "cases")
+
+# longer streams on larger inputs: 2000 draws from each of five weight vectors, a fifth of the items zero
+rng = np.random.default_rng(11)
+arrays = {}
+sizes = (1, 2, 33, 1000, 20000)
+for n in sizes:
+    w = rng.uniform(0.0, 3.0, n).astype(np.float32)
+    w[rng.integers(0, n, n // 5)] = 0.0
+    if w.sum() == 0:
+        w[0] = 1.0
+    arrays["weights_%d" % n] = w
+    arrays["draws_%d" % n] = o.RefWeightedSampler(w).draw(2000)
+out = os.path.join(os.path.dirname(os.path.abspath(__file__)), "weighted_sampler_draws.npz")
+np.savez_compressed(out, sizes=np.array(sizes, np.int32), **arrays)
+print("wrote", out, len(sizes), "weight vectors")

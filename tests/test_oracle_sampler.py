@@ -1,5 +1,5 @@
 """WeightedSampler restatement (oracle/vg_oracle.c vgo_sampler_*) pinned against the REFERENCE's own
-code: golden vectors generated from voxgraph::WeightedSampler compiled out of /root/reference
+code: golden vectors generated from voxgraph::WeightedSampler compiled out of the reference sources
 (tests/golden/make_sampler_golden.py), and - where oracle/_ref is present - the compiled reference
 itself."""
 import json
@@ -11,6 +11,7 @@ import pytest
 from oracle import oracle as o
 
 GOLDEN = os.path.join(os.path.dirname(__file__), "golden", "weighted_sampler.json")
+REF_DRAWS = os.path.join(os.path.dirname(__file__), "golden", "weighted_sampler_draws.npz")
 
 
 def _cases():
@@ -43,17 +44,15 @@ def test_draws_match_reference_golden(case):
 
 
 def test_draws_match_compiled_reference():
-    if o.ref_sampler_lib() is None:
-        pytest.skip("oracle/_ref/libvgref_sampler.so not built (no /root/reference)")
-    rng = np.random.default_rng(11)
-    for n in (1, 2, 33, 1000, 20000):
-        w = rng.uniform(0.0, 3.0, n).astype(np.float32)
-        w[rng.integers(0, n, n // 5)] = 0.0
-        if w.sum() == 0:
-            w[0] = 1.0
-        a = o.WeightedSampler(w).draw(2000)
-        b = o.RefWeightedSampler(w).draw(2000)
-        assert np.array_equal(a, b)
+    """2000 draws from each of five weight vectors (1 to 20000 items) as the compiled reference made
+    them (tests/golden/weighted_sampler_draws.npz); where oracle/_ref is built, also the live one."""
+    z = np.load(REF_DRAWS)
+    live = o.ref_sampler_lib() is not None
+    for n in z["sizes"]:
+        w, want = z["weights_%d" % n], z["draws_%d" % n]
+        assert np.array_equal(o.WeightedSampler(w).draw(len(want)), want)
+        if live:
+            assert np.array_equal(o.RefWeightedSampler(w).draw(len(want)), want)
 
 
 def test_zero_weight_items_are_never_drawn_and_frequencies_follow_weights():
